@@ -4,6 +4,9 @@
   python bench.py --gpus N --steps K --warmup W                      # this repo's CUDA path, BASELINE configs[1]
   python bench.py --config 3|4|5 [--scaling strong] ...              # the other BASELINE configs (see CONFIGS)
   python bench.py --impl reference --gpus N --steps K ...            # the reference's CPU path on the host cores
+  python bench.py ... --dump-outputs DIR                             # also write the arrays the last timed step returned
+                                                                     # (the sample; for config 5 also the trajectories) to
+                                                                     # DIR/<name>.npy, float32; the inputs are seeded
 
 One bench "step" = one full sampling call of the workload on every rank (config 2: SMPL diffusion, 100 DDPM steps,
 B=64, T=30, inpainted past of 10 frames); the metric counts the DENOISING steps executed.
@@ -292,10 +295,12 @@ def run_ours(args):
         rollout = RolloutDriver(eng, past_len=c["past"], n_windows=c["windows"] - 1)
 
     def one_call():
+        """one sampling call; returns what its caller receives: the sample, and for the rollout the world-coordinate
+        trajectories as well"""
         if rollout is None:
-            eng.p_sample_loop(tape_d, gt_d, mask_d, correction=c["correction"], use_graph=True, out=out)
-        else:
-            rollout.run(tape_d, gt_d, mask_d, torch.from_numpy(b["hand_pose"]).to(dev), torch.from_numpy(b["betas"]).to(dev), out)
+            return dict(sample=eng.p_sample_loop(tape_d, gt_d, mask_d, correction=c["correction"], use_graph=True, out=out))
+        traj = rollout.run(tape_d, gt_d, mask_d, torch.from_numpy(b["hand_pose"]).to(dev), torch.from_numpy(b["betas"]).to(dev), out)
+        return dict(sample=out, **traj)
 
     def barrier():
         if world > 1:
@@ -314,10 +319,13 @@ def run_ours(args):
     for s, e in ev:
         flush.fill_(1.0)  # evict L2 between timed iterations (outside the event pair)
         s.record()
-        one_call()
+        result = one_call()
         e.record()
     barrier()
     wall = time.perf_counter() - wall0
+    if args.dump_outputs:
+        # host copies now: the legs below reuse the device buffers
+        dump = {k: v.detach().cpu().numpy() for k, v in result.items()}
     launches = eng.launch_count - l0
     dev_ms = sum(s.elapsed_time(e) for s, e in ev)
     # ---- end-to-end leg through the public API with host buffers
@@ -434,15 +442,26 @@ def run_ours(args):
             line["cpu_baseline"] = dict(value=r["rate"], unit=UNIT, cores=r["cores"], kind=r["kind"], sample=r["sample"],
                                         plain_step_s=r["plain_s"], correction_step_extra_s=r["corr_s"])
         print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dump, rank if world > 1 else None)
     if world > 1:
         dist.destroy_process_group()
     eng.close()
 
 
+def dump_outputs(directory, arrays, rank=None):
+    """<directory>/<name>.npy (float32) of each array of the last timed step, <name>_rank<r>.npy for multi-rank runs:
+    two builds run with the same arguments sample the same inputs, so their files compare output for output"""
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20, "outputs above 64 MB: dump a sample instead"
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ("" if rank is None else "_rank%d" % rank) + ".npy"), a.astype(np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed sampling calls (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS))
@@ -450,7 +469,13 @@ def main():
     ap.add_argument("--backend", default=None, choices=[None, "simt", "tcgen05"])
     ap.add_argument("--cpu-steps", type=int, default=6)
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the last timed step returned to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

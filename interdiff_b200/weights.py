@@ -137,13 +137,14 @@ REF_WEIGHT_DIR = os.environ.get("INTERDIFF_B200_WEIGHTS") or os.path.join(
     os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "weights_ref")
 
 
-def ref_weights_path(name):
-    return os.path.join(REF_WEIGHT_DIR, name + ".npz")
+def ref_weights_path(name, directory=None):
+    return os.path.join(directory or REF_WEIGHT_DIR, name + ".npz")
 
 
-def load_ref_weights(name):
-    """Returns {name: ndarray} exported by oracle/export_ref_weights.py, or None if absent."""
-    p = ref_weights_path(name)
+def load_ref_weights(name, directory=None):
+    """Returns {name: ndarray} exported by oracle/export_ref_weights.py into `directory` (default REF_WEIGHT_DIR),
+    or None if absent."""
+    p = ref_weights_path(name, directory)
     if not os.path.exists(p):
         return None
     with np.load(p) as z:

@@ -8,12 +8,11 @@ may import this package.  The product package (interdiff_b200/) never imports it
 fails loudly when its CUDA library is missing.
 
 Pinning status (see DESIGN.md "Oracle"):
-  * oracle.restate (the restatement that travels to the GPU box) is checked in
-    tests/test_oracle_vs_reference.py against the reference's OWN classes
-    (interdiff/model, interdiff/diffusion, interdiff/libsmpl, interdiff/data/tools.py,
-    interdiff/tools.py) imported from /root/reference through oracle.shims, with the shipped
-    checkpoints; and against golden vectors generated from those classes
-    (oracle/make_golden.py -> tests/golden/*.npz).
+  * oracle.restate is checked in tests/test_oracle_vs_reference.py and tests/test_golden.py
+    against golden vectors generated from the reference's OWN classes (interdiff/model,
+    interdiff/diffusion, interdiff/libsmpl, interdiff/data/tools.py, interdiff/tools.py)
+    imported from the reference tree through oracle.shims (oracle/make_golden.py ->
+    tests/golden/).
   * Third-party arithmetic whose source is NOT under /root/reference is restated from the
     published algorithm and is "parity unpinned" at that boundary:
       - local_attention.LocalAttention (unpinned version; both rotary placements kept,

@@ -129,12 +129,18 @@ def build_obj_projector(state_dict=None, past_len=10, future_len=20):
     return model, args
 
 
-def build_obj_projector_skeleton():
-    """Reference skeleton correction net (model/correction_skeleton.py:8-135) with checkpoints/obj_skeleton.ckpt."""
+def build_obj_projector_skeleton(state_dict=None):
+    """Reference skeleton correction net (model/correction_skeleton.py:8-135) with checkpoints/obj_skeleton.ckpt
+    (state_dict=None) or a caller-provided state dict (BatchNorm batch counters may be omitted)."""
     m = modules()["model.correction_skeleton"]
     hp, sd = load_ckpt("obj_skeleton")
     model = m.ObjProjector(Namespace(**hp))
-    model.load_state_dict(sd, strict=True)
+    if state_dict is None:
+        model.load_state_dict(sd, strict=True)
+    else:
+        sd = state_dict
+        missing, unexpected = model.load_state_dict(sd, strict=False)
+        assert not unexpected and all(k.endswith("num_batches_tracked") for k in missing), (missing, unexpected)
     model.eval()
     return model, Namespace(**hp), sd
 

@@ -7,9 +7,8 @@ Every function cites the reference file:line it follows (paths relative to
 /root/reference/interdiff).  Weights are passed as flat dicts {reference state_dict name:
 tensor} so that the same dict feeds the reference module, this restatement and the CUDA path.
 
-Pinned by tests/test_oracle_vs_reference.py (runs where /root/reference exists) and by the
-golden vectors under tests/golden/ (generated from the reference's own classes by
-oracle/make_golden.py).
+Pinned by the golden vectors under tests/golden/ (generated from the reference's own classes by
+oracle/make_golden.py; tests/test_oracle_vs_reference.py and tests/test_golden.py).
 """
 import math
 

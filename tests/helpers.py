@@ -5,6 +5,7 @@ import torch
 from interdiff_b200 import synthetic as S
 from interdiff_b200 import weights as W
 from oracle import restate as R
+from oracle.export_ref_weights import OUT_DIR as REF_WEIGHTS
 
 
 def rel(a, b):
@@ -19,7 +20,7 @@ def mdm_weights(variant="smpl", source="auto", seed=233):
     shapes = W.mdm_hot_shapes(variant, F=F)
     sd = None
     if source in ("ref", "auto"):
-        sd = W.load_ref_weights("diffusion_" + variant)
+        sd = W.load_ref_weights("diffusion_" + variant, REF_WEIGHTS)
         if sd is None and source == "ref":
             import pytest
             pytest.skip("exported reference weights not present (oracle/export_ref_weights.py)")
@@ -38,7 +39,7 @@ def encoder_weights(source="auto", seed=234):
     sd = mdm_weights("smpl", source)
     enc = None
     if source in ("ref", "auto"):
-        enc = W.load_ref_weights("diffusion_smpl_encoder")
+        enc = W.load_ref_weights("diffusion_smpl_encoder", REF_WEIGHTS)
         if enc is None and source == "ref":
             import pytest
             pytest.skip("exported encoder weights not present (oracle/export_ref_weights.py)")
@@ -52,7 +53,7 @@ def encoder_weights(source="auto", seed=234):
 def projector_weights(source="auto", seed=233):
     sd = None
     if source in ("ref", "auto"):
-        sd = W.load_ref_weights("correction_smpl")
+        sd = W.load_ref_weights("correction_smpl", REF_WEIGHTS)
         if sd is None and source == "ref":
             import pytest
             pytest.skip("exported reference weights not present")
@@ -64,7 +65,7 @@ def projector_weights(source="auto", seed=233):
 def projector_skeleton_weights(source="auto", seed=235):
     sd = None
     if source in ("ref", "auto"):
-        sd = W.load_ref_weights("correction_skeleton")
+        sd = W.load_ref_weights("correction_skeleton", REF_WEIGHTS)
         if sd is None and source == "ref":
             import pytest
             pytest.skip("exported reference weights not present")

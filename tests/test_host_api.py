@@ -1,6 +1,8 @@
 """CPU-side checks of the drop-in boundary: the C ABI exports every symbol the header declares,
 the mirrored modules load the reference checkpoints strictly, the diffusion tables equal the
 reference's, and the product path refuses to run without a GPU (no CPU fallback)."""
+import gzip
+import json
 import os
 import re
 from argparse import Namespace
@@ -11,10 +13,19 @@ import torch
 
 from interdiff_b200 import _lib
 from interdiff_b200 import weights as W
-from oracle import ref_loader as RL
 from oracle import restate as R
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+
+
+def reference_checkpoint(name):
+    """(hyper_parameters, {state_dict name: zero tensor of the stored shape}) of the reference's shipped checkpoint `name`
+    (tests/golden/checkpoints.json.gz, written by `python -m oracle.make_golden --reference-checks`)"""
+    with gzip.open(os.path.join(GOLDEN, "checkpoints.json.gz")) as f:
+        ck = json.load(f)[name]
+    return ck["hyper_parameters"], {k: torch.zeros(shape) for k, shape in ck["state_dict"].items()}
+
 
 SMPL_ARGS = dict(embedding_dim=256, smpl_dim=132, use_pointnet2=1, dropout=0.0, num_heads=4, ff_size=1024, activation="gelu",
                  latent_usage="memory", future_len=25, past_len=10, cond_mask_prob=0, diffusion_steps=1000, noise_schedule="cosine",
@@ -59,17 +70,16 @@ def test_mirror_state_dict_names_match_tables():
         assert k in psd and tuple(psd[k].shape) == tuple(shp), k
 
 
-@pytest.mark.skipif(not RL.available(), reason="reference tree not present")
 def test_mirrors_load_reference_checkpoints_strictly():
     from interdiff_b200.model import correction_smpl, diffusion_skeleton, diffusion_smpl
-    hp, sd = RL.load_ckpt("diffusion")
+    hp, sd = reference_checkpoint("diffusion")
     m, d = diffusion_smpl.create_model_and_diffusion(Namespace(**hp))
     m.load_state_dict(sd, strict=True)
     assert d.num_timesteps == 1000
-    hp, sd = RL.load_ckpt("diffusion_skeleton")
+    hp, sd = reference_checkpoint("diffusion_skeleton")
     m, _ = diffusion_skeleton.create_model_and_diffusion(Namespace(**hp))
     m.load_state_dict(sd, strict=True)
-    hp, sd = RL.load_ckpt("correction")
+    hp, sd = reference_checkpoint("correction")
     p = correction_smpl.ObjProjector(Namespace(**{**hp, "dct": 10}))
     p.load_state_dict(sd, strict=True)
 
@@ -88,23 +98,17 @@ def test_diffusion_tables_and_spacing():
     d = SpacedDiffusion(use_timesteps=space_timesteps(1000, [100]), betas=gd.get_named_beta_schedule("cosine", 1000),
                         model_mean_type=gd.ModelMeanType.START_X, model_var_type=gd.ModelVarType.FIXED_SMALL, loss_type=gd.LossType.MSE)
     assert d.num_timesteps == 100 and d.timestep_map[0] == 0 and d.timestep_map[-1] == 999
-    if RL.available():
-        ref = RL.modules()["diffusion.respace"]
-        assert ref.space_timesteps(1000, [100]) == space_timesteps(1000, [100])
-        assert ref.space_timesteps(300, "10,15,20") == space_timesteps(300, "10,15,20")
-        rd = ref.SpacedDiffusion(use_timesteps=ref.space_timesteps(1000, [100]), betas=gd.get_named_beta_schedule("cosine", 1000),
-                                 model_mean_type=RL.modules()["diffusion.gaussian_diffusion"].ModelMeanType.START_X,
-                                 model_var_type=RL.modules()["diffusion.gaussian_diffusion"].ModelVarType.FIXED_SMALL,
-                                 loss_type=RL.modules()["diffusion.gaussian_diffusion"].LossType.MSE)
-        assert np.array_equal(rd.betas, d.betas) and rd.timestep_map == d.timestep_map
+    # the reference's diffusion.respace on the same arguments (tests/golden/reference_checks.npz)
+    ref = np.load(os.path.join(GOLDEN, "reference_checks.npz"))
+    assert space_timesteps(1000, [100]) == set(ref["space_1000_100"].tolist())
+    assert space_timesteps(300, "10,15,20") == set(ref["space_300_10_15_20"].tolist())
+    assert np.array_equal(ref["spaced_1000_100_betas"], d.betas) and ref["spaced_1000_100_timestep_map"].tolist() == d.timestep_map
 
 
 def test_skeleton_projector_mirror_loads_checkpoint_strictly():
     """interdiff_b200.model.correction_skeleton.ObjProjector carries the reference's state_dict names (obj_skeleton.ckpt)"""
-    if not RL.available():
-        pytest.skip("reference tree not present")
     from interdiff_b200.model.correction_skeleton import ObjProjector
-    hp, sd = RL.load_ckpt("obj_skeleton")
+    hp, sd = reference_checkpoint("obj_skeleton")
     m = ObjProjector(Namespace(**hp))
     missing, unexpected = m.load_state_dict(sd, strict=True)
     assert not missing and not unexpected
