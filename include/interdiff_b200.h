@@ -86,6 +86,17 @@ int idb_denoiser_forward(idb_handle* h, const float* x, const int64_t* timesteps
  *   cond_out     (Tp,B,256)  sequence-first like the reference; feed it to idb_denoiser_bind */
 int idb_encode_condition(idb_handle* h, int B, int Tp, const float* past, const float* pc_embedding, float* cond_out, void* stream);
 
+/* Conditioning encoder of the skeleton model (variant 1) = MDM._get_embeddings after the `gt` concatenation (reference
+ * model/diffusion_skeleton.py:194-215):
+ *   cond = encoder(PositionalEmbedding(bodyEmbedding(body_past) + objEmbedding(obj_past) + shapeEmbedding(zero_pose_obj)))
+ * Needs the "encoder.layers.*" (d_ff 256) and "shapeEmbedding.*" tensors loaded before idb_denoiser_commit.
+ *   past          (B,1,C,Tp)        the first past_len frames of the sample tensor, C = 3 n_joints + 3 n_points + 7 (the 7 pose
+ *                                   channels are not embedded, as in the reference)
+ *   zero_pose_obj (B,n_points,3)    canonical object keypoints (model_kwargs['zero_pose_obj'])
+ *   cond_out      (Tp,B,256)        sequence-first like the reference; feed it to idb_denoiser_bind */
+int idb_encode_condition_skeleton(idb_handle* h, int B, int Tp, const float* past, const float* zero_pose_obj, float* cond_out,
+                                  void* stream);
+
 /* PointNet++ (MSG) point-cloud encoder = MDM.pcEmbedding, PointNet2Encoder(c_in=1, c_out=256, num_keypoints=1)
  * (reference model/layers.py:111-175, called at model/diffusion_smpl.py:210-211); the furthest-point-sampling /
  * ball-query / grouping operators of the un-vendored pointnet2_ops 3.0.0 are rebuilt for sm_100a.
@@ -188,6 +199,15 @@ int idb_correction_set_log(idb_handle* h, uint8_t* cond_log, int32_t* contact_lo
 int idb_metrics(idb_handle* h, int T, int B, int J, int P, int Db, const float* obj_pred, const float* body_jtr, const float* body,
                 const float* obj_gt, const float* body_jtr_gt, const float* body_gt, const float* verts, const float* obj_points,
                 float* out, void* stream);
+
+/* Evaluation metrics of the skeleton model, per sample, on the device (reference eval_skeleton.py:46-68 calc_metric_single and
+ * train_diffusion_skeleton.py:65-87 calc_metric, which average the same terms over the whole batch):
+ *   pred / gt (B,1,3 n_joints + 3 n_points + 7,T) in the sample layout, channels [joints | object keypoints | trans(3), quat xyzw(4)]
+ *   out [5][B]: means over the future frames t >= past_len of mpjpe_h (L2 over joints), mpjpe_o (L2 over keypoints),
+ *   translation_error, rotation_error (min over the quaternion sign of the L1 distance, eval_skeleton.py) and
+ *   rotation_error_l2 (the same with the L2 norm, train_diffusion_skeleton.py). */
+int idb_skeleton_metrics(idb_handle* h, int B, int T, int past_len, int n_joints, int n_points, const float* pred, const float* gt,
+                         float* out, void* stream);
 
 /* Post-processing of a sampled window: `smooth` (eval_smpl_short.py:217-223) in place on x (T, inner) - every future frame is
  * shifted by 2 x[-F-1] - x[-F-2] - x[-F] (old values) - and the element-wise minimum that reduces the metric vectors of the

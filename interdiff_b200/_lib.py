@@ -25,6 +25,8 @@ _SIGS = {
     "idb_last_error": (C.c_char_p, [_P]),
     "idb_launch_count": (C.c_longlong, [_P]),
     "idb_encode_condition": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P, _P]),
+    "idb_encode_condition_skeleton": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P, _P]),
+    "idb_skeleton_metrics": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P]),
     "idb_pointcloud_embed": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P]),
     "idb_metrics": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "idb_rollout_next_window": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]),

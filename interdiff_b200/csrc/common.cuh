@@ -67,6 +67,7 @@ struct Denoiser {
     __half *e_xtok_b = nullptr, *e_xtok_s = nullptr, *e_h_b = nullptr, *e_h_s = nullptr, *e_h2_b = nullptr, *e_h2_s = nullptr,
            *e_ff_b = nullptr, *e_ff_s = nullptr;
     std::vector<void*> enc_owned;
+    float *w_shapeT = nullptr, *b_shape = nullptr;   // skeleton: shapeEmbedding k-major [3 n_points][D] + bias (null unless loaded)
     // PointNet++ point-cloud encoder (pointnet.cu): folded weights + workspace; optional like the encoder
     bool pn_ready = false; int pn_cap = 0;
     float *pn_w1 = nullptr, *pn_w2 = nullptr, *pn_xyz1 = nullptr, *pn_feat1 = nullptr;

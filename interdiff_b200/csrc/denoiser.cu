@@ -1237,9 +1237,10 @@ extern "C" int idb_denoiser_load(idb_handle* h, const char* name, const float* d
     Denoiser& d = h->den;
     if (!d.configured) return idb_fail(h, IDB_ERR_STATE, "idb_denoiser_init first");
     std::string s(name);
-    // tensors of the sampling hot path and, when given, of the conditioning encoder (PointNet++ is a later row)
+    // tensors of the sampling hot path and, when given, of the conditioning encoder (PointNet++ for SMPL, shapeEmbedding for
+    // the skeleton model)
     bool want = s.rfind("decoder.layers.", 0) == 0 || s.rfind("encoder.layers.", 0) == 0 || s.rfind("pcEmbedding.", 0) == 0 ||
-                s.rfind("bodyEmbedding.", 0) == 0 || s.rfind("objEmbedding.", 0) == 0 ||
+                s.rfind("shapeEmbedding.", 0) == 0 || s.rfind("bodyEmbedding.", 0) == 0 || s.rfind("objEmbedding.", 0) == 0 ||
                 s.rfind("bodyFinalLinear.", 0) == 0 || s.rfind("objFinalLinear.", 0) == 0 ||
                 s.rfind("embedTimeStep.time_embed.", 0) == 0 || s == "PositionalEmbedding.pe";
     if (!want || s.find("inv_freq") != std::string::npos) return IDB_OK;
@@ -1445,10 +1446,19 @@ extern "C" int idb_denoiser_commit(idb_handle* h) {
     }
     // conditioning encoder (optional: present when its tensors were loaded; SURVEY 8f rank 1)
     d.enc_layers.clear();
+    d.w_shapeT = d.b_shape = nullptr;
     if (d.raw.count("encoder.layers.0.linear1.weight")) {
         for (int l = 0; l < c.n_layers; l++) {
             const int rc = build_layer("encoder.layers.", l, false, d.enc_layers);
             if (rc) return rc;
+        }
+        if (c.variant == 1) {
+            // skeleton: the object-shape embedding of the canonical keypoints (model/diffusion_skeleton.py:203), k-major
+            GET(ws, "shapeEmbedding.weight", D, c.c_obj) GET(bs, "shapeEmbedding.bias", D)
+            auto hws = P.host(ws);
+            std::vector<float> wT((size_t)c.c_obj * D);
+            for (int n = 0; n < D; n++) for (int k = 0; k < c.c_obj; k++) wT[(size_t)k * D + n] = hws[(size_t)n * c.c_obj + k];
+            d.w_shapeT = P.up(wT); d.b_shape = bs->p;
         }
     }
 #undef GET
@@ -1805,9 +1815,10 @@ int idb_denoiser_prepare_kernels(idb_handle* h) {
 // ---------------------------------------------------------------------------------------------
 // Conditioning encoder (SURVEY 8f rank 1, the part of MDM._get_embeddings after the point-cloud encoder,
 // model/diffusion_smpl.py:217-221): cond = encoder(PositionalEmbedding(bodyEmbedding(past body) +
-// objEmbedding(past obj) + pc_embedding)).  Runs once per batch before idb_denoiser_bind; the layers reuse the
+// objEmbedding(past obj) + pc_embedding)); for the skeleton model (model/diffusion_skeleton.py:194-215) the
+// point-cloud term is shapeEmbedding(zero_pose_obj).  Runs once per batch before idb_denoiser_bind; the layers reuse the
 // decoder's kernels (folded-QKV GEMM + k_attn_ln, the QaN kernel without its cross-attention half, the fused
-// feed-forward kernel), rows m = b*Tp + t.
+// feed-forward kernel or, for d_ff != 1024, two GEMMs), rows m = b*Tp + t.  Only the token kernels differ per variant.
 namespace {
 
 // past (B,1,C,Tp) -> token pairs [B*Tp][Cp] (zero padded) + addend[b*Tp+t][:] = (pc[b] + b_body + b_obj) + pe[t]
@@ -1846,40 +1857,61 @@ __global__ void k_ln_seq_first(const float* __restrict__ a, const float* __restr
     }
 }
 
+// skeleton variant (model/diffusion_skeleton.py:194-215): past (B,1,C,Tp) with C = 3 n_joints + 3 n_points + 7 -> token pairs
+// [B*Tp][Cp] (zero padded; W_in has zero rows for the 7 pose channels, so the whole past slice is fed as it is) and
+// addend[b*Tp+t][:] = (shape[b] + b_body + b_obj) + pe[t], shape[b] = shapeEmbedding(zero_pose_obj[b]) = Ws zp[b] + bs
+// (K = 3 n_points fp32 terms per output, ascending k).  grid B, block D, dynamic shared memory K floats.
+__global__ void __launch_bounds__(D)
+k_skel_cond_tokens(const float* __restrict__ past, const float* __restrict__ zp, const float* __restrict__ wsT, const float* __restrict__ bs,
+                   const float* __restrict__ b_in, const float* __restrict__ pe, __half* __restrict__ xtok_b, __half* __restrict__ xtok_s,
+                   float* __restrict__ add, int C, int Cp, int Tp, int K) {
+    extern __shared__ float s_zp[];
+    const int b = blockIdx.x, n = threadIdx.x;
+    for (int k = n; k < K; k += D) s_zp[k] = zp[(size_t)b * K + k];
+    for (int i = n; i < Tp * Cp; i += D) {
+        const int t = i / Cp, c = i % Cp;
+        const size_t o = ((size_t)b * Tp + t) * Cp + c;
+        split_f16(c < C ? past[((size_t)b * C + c) * Tp + t] : 0.f, xtok_b[o], xtok_s[o]);
+    }
+    __syncthreads();
+    float s = 0.f;
+    for (int k = 0; k < K; k++) s = fmaf(wsT[(size_t)k * D + n], s_zp[k], s);
+    const float base = (s + bs[n]) + b_in[n];
+    for (int t = 0; t < Tp; t++) add[((size_t)b * Tp + t) * D + n] = base + pe[(size_t)t * D + n];
+}
+
 }  // namespace
 
-extern "C" int idb_encode_condition(idb_handle* h, int B, int Tp, const float* past, const float* pc_embedding, float* cond_out,
-                                    void* stream) {
-    IDB_ENTER(h);
-    if (!h || !past || !pc_embedding || !cond_out || B <= 0 || Tp <= 0) return IDB_ERR_ARG;
+// encoder workspace for M = B*Tp rows (token pairs Cp wide), grown on demand
+static int encoder_workspace(idb_handle* h, int M, int Cp) {
     Denoiser& d = h->den;
-    if (!d.committed) return idb_fail(h, IDB_ERR_STATE, "idb_denoiser_commit first");
-    if (d.enc_layers.empty()) return idb_fail(h, IDB_ERR_STATE, "the conditioning encoder's weights (encoder.layers.*) were not loaded");
-    if (Tp > 36) return idb_fail(h, IDB_ERR_ARG, "supported past window: <= 36 frames");
+    const int F = d.cfg.d_ff, H = d.cfg.n_heads;
+    if (M <= d.enc_cap) return IDB_OK;
+    for (void* p : d.enc_owned) cudaFree(p);
+    d.enc_owned.clear();
+    d.enc_cap = 0;
+    auto A = [&](float** p, size_t n) { if (cudaMalloc((void**)p, n * sizeof(float)) != cudaSuccess) return 1; d.enc_owned.push_back(*p); return 0; };
+    auto AH = [&](__half** p, size_t n) { if (cudaMalloc((void**)p, n * sizeof(__half)) != cudaSuccess) return 1; d.enc_owned.push_back(*p); return 0; };
+    int rc = 0;
+    rc |= A(&d.e_add, (size_t)M * D); rc |= A(&d.e_h, (size_t)M * D); rc |= A(&d.e_h2, (size_t)M * D); rc |= A(&d.e_z, (size_t)M * D);
+    rc |= A(&d.e_qkv, (size_t)M * (2 * D + H * D));
+    rc |= AH(&d.e_xtok_b, (size_t)M * Cp); rc |= AH(&d.e_xtok_s, (size_t)M * Cp);
+    rc |= AH(&d.e_h_b, (size_t)M * D); rc |= AH(&d.e_h_s, (size_t)M * D); rc |= AH(&d.e_h2_b, (size_t)M * D); rc |= AH(&d.e_h2_s, (size_t)M * D);
+    rc |= AH(&d.e_ff_b, (size_t)M * F); rc |= AH(&d.e_ff_s, (size_t)M * F);
+    if (rc) return idb_fail(h, IDB_ERR_CUDA, "out of device memory (encoder workspace)");
+    d.enc_cap = M;
+    return IDB_OK;
+}
+
+// Shared by both conditioning entry points, on the prepared token pairs (e_xtok, Cp wide) and addend (e_add): input embedding
+// GEMM, the encoder layer stack, the last norm into the sequence-first (Tp,B,D) output.
+static int encoder_stack(idb_handle* h, int B, int Tp, int Cp, float* cond_out, cudaStream_t st) {
+    Denoiser& d = h->den;
     const idb_denoiser_config& c = d.cfg;
-    const int M = B * Tp, F = c.d_ff, H = c.n_heads, N = c.n_queries, C = c.c_body + c.c_obj, Cp = (C + 7) & ~7;
-    if (c.variant != 0) return idb_fail(h, IDB_ERR_ARG, "idb_encode_condition: SMPL model only");
-    cudaStream_t st = (cudaStream_t)stream;
+    const int M = B * Tp, F = c.d_ff, H = c.n_heads, N = c.n_queries;
     const bool fused = h->gemm_backend == 1 && h->fused_mlp && idb_mlp_tcgen05_supported(D, F);
-    if (M > d.enc_cap) {
-        for (void* p : d.enc_owned) cudaFree(p);
-        d.enc_owned.clear();
-        d.enc_cap = 0;
-        auto A = [&](float** p, size_t n) { if (cudaMalloc((void**)p, n * sizeof(float)) != cudaSuccess) return 1; d.enc_owned.push_back(*p); return 0; };
-        auto AH = [&](__half** p, size_t n) { if (cudaMalloc((void**)p, n * sizeof(__half)) != cudaSuccess) return 1; d.enc_owned.push_back(*p); return 0; };
-        int rc = 0;
-        rc |= A(&d.e_add, (size_t)M * D); rc |= A(&d.e_h, (size_t)M * D); rc |= A(&d.e_h2, (size_t)M * D); rc |= A(&d.e_z, (size_t)M * D);
-        rc |= A(&d.e_qkv, (size_t)M * (2 * D + H * D));
-        rc |= AH(&d.e_xtok_b, (size_t)M * Cp); rc |= AH(&d.e_xtok_s, (size_t)M * Cp);
-        rc |= AH(&d.e_h_b, (size_t)M * D); rc |= AH(&d.e_h_s, (size_t)M * D); rc |= AH(&d.e_h2_b, (size_t)M * D); rc |= AH(&d.e_h2_s, (size_t)M * D);
-        rc |= AH(&d.e_ff_b, (size_t)M * F); rc |= AH(&d.e_ff_s, (size_t)M * F);
-        if (rc) return idb_fail(h, IDB_ERR_CUDA, "out of device memory (encoder workspace)");
-        d.enc_cap = M;
-    }
     const bool pdl = h->pdl != 0;
     int rc;
-    k_cond_tokens<<<B, 256, 0, st>>>(past, pc_embedding, d.b_in, d.pe, d.e_xtok_b, d.e_xtok_s, d.e_add, C, Cp, Tp);
-    LAUNCH_CHECK(h);
     if ((rc = linear(h, d.e_xtok_b, d.e_xtok_s, Cp, d.w_in_b, d.w_in_s, Cp, nullptr, d.e_add, d.e_h, d.e_h_b, d.e_h_s, D, M, D, Cp, EPI_RES, st)))
         return rc;
     const dim3 slab_grid(B, (Tp + SLAB - 1) / SLAB);
@@ -1917,6 +1949,7 @@ extern "C" int idb_encode_condition(idb_handle* h, int B, int Tp, const float* p
             if ((rc = idb_mlp_tcgen05(h, d.e_h2_b, d.e_h2_s, L.w1_b, L.w1_s, L.b1, L.w2_b, L.w2_s, L.b2, d.e_h2, D, d.e_z, D, M, h->pdl, st)))
                 return rc;
         } else {
+            // two GEMMs (also the only path for d_ff != 1024, e.g. the skeleton model's 256)
             if ((rc = linear(h, d.e_h2_b, d.e_h2_s, D, L.w1_b, L.w1_s, D, L.b1, nullptr, nullptr, d.e_ff_b, d.e_ff_s, F, M, F, D,
                              EPI_BIAS | EPI_GELU, st))) return rc;
             if ((rc = linear(h, d.e_ff_b, d.e_ff_s, F, L.w2_b, L.w2_s, F, L.b2, d.e_h2, d.e_z, nullptr, nullptr, D, M, D, F, EPI_BIAS | EPI_RES, st)))
@@ -1929,6 +1962,46 @@ extern "C" int idb_encode_condition(idb_handle* h, int B, int Tp, const float* p
                pending ? pending->ln3b : (const float*)nullptr, cond_out, B, Tp);
     LAUNCH_CHECK(h);
     return IDB_OK;
+}
+
+extern "C" int idb_encode_condition(idb_handle* h, int B, int Tp, const float* past, const float* pc_embedding, float* cond_out,
+                                    void* stream) {
+    IDB_ENTER(h);
+    if (!h || !past || !pc_embedding || !cond_out || B <= 0 || Tp <= 0) return IDB_ERR_ARG;
+    Denoiser& d = h->den;
+    if (!d.committed) return idb_fail(h, IDB_ERR_STATE, "idb_denoiser_commit first");
+    if (d.enc_layers.empty()) return idb_fail(h, IDB_ERR_STATE, "the conditioning encoder's weights (encoder.layers.*) were not loaded");
+    if (Tp > 36) return idb_fail(h, IDB_ERR_ARG, "supported past window: <= 36 frames");
+    const idb_denoiser_config& c = d.cfg;
+    const int M = B * Tp, C = c.c_body + c.c_obj, Cp = (C + 7) & ~7;
+    if (c.variant != 0) return idb_fail(h, IDB_ERR_ARG, "idb_encode_condition: SMPL model only (skeleton: idb_encode_condition_skeleton)");
+    cudaStream_t st = (cudaStream_t)stream;
+    int rc;
+    if ((rc = encoder_workspace(h, M, Cp))) return rc;
+    k_cond_tokens<<<B, 256, 0, st>>>(past, pc_embedding, d.b_in, d.pe, d.e_xtok_b, d.e_xtok_s, d.e_add, C, Cp, Tp);
+    LAUNCH_CHECK(h);
+    return encoder_stack(h, B, Tp, Cp, cond_out, st);
+}
+
+extern "C" int idb_encode_condition_skeleton(idb_handle* h, int B, int Tp, const float* past, const float* zero_pose_obj, float* cond_out,
+                                             void* stream) {
+    IDB_ENTER(h);
+    if (!h || !past || !zero_pose_obj || !cond_out || B <= 0 || Tp <= 0) return IDB_ERR_ARG;
+    Denoiser& d = h->den;
+    if (!d.committed) return idb_fail(h, IDB_ERR_STATE, "idb_denoiser_commit first");
+    const idb_denoiser_config& c = d.cfg;
+    if (c.variant != 1) return idb_fail(h, IDB_ERR_ARG, "idb_encode_condition_skeleton: skeleton model only (SMPL: idb_encode_condition)");
+    if (d.enc_layers.empty() || !d.w_shapeT)
+        return idb_fail(h, IDB_ERR_STATE, "the conditioning encoder's weights (encoder.layers.*, shapeEmbedding.*) were not loaded");
+    if (Tp > 36 || Tp > d.pe_rows) return idb_fail(h, IDB_ERR_ARG, "supported past window: <= 36 frames");
+    const int M = B * Tp, C = c.c_body + c.c_obj + c.c_extra, Cp = (C + 7) & ~7, K = c.c_obj;
+    cudaStream_t st = (cudaStream_t)stream;
+    int rc;
+    if ((rc = encoder_workspace(h, M, Cp))) return rc;
+    k_skel_cond_tokens<<<B, D, K * sizeof(float), st>>>(past, zero_pose_obj, d.w_shapeT, d.b_shape, d.b_in, d.pe, d.e_xtok_b, d.e_xtok_s,
+                                                        d.e_add, C, Cp, Tp, K);
+    LAUNCH_CHECK(h);
+    return encoder_stack(h, B, Tp, Cp, cond_out, st);
 }
 
 extern "C" int idb_denoiser_forward(idb_handle* h, const float* x, const int64_t* timesteps, float* out, void* stream) {

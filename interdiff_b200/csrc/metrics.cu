@@ -3,6 +3,7 @@
 // ambiguity resolved by the minimum) and the penetration ratio of the posed object points against the body mesh.
 // The penetration term reuses the hot path's kernels (vertex normals, cluster-pruned signed nearest neighbour);
 // everything else is one reduction kernel per batch.  All reductions run in a fixed order (bit-reproducible).
+// The skeleton model's metrics (eval_skeleton.py:46-68, train_diffusion_skeleton.py:65-87) are one kernel of their own.
 #include "common.cuh"
 #include "body.cuh"
 
@@ -122,6 +123,66 @@ extern "C" int idb_metrics(idb_handle* h, int T, int B, int J, int P, int Db, co
     if ((rc = idb_vertex_normals(h, F, verts, normals, st))) return rc;
     if ((rc = idb_signed_nn(h, F, P, V, objp, verts, normals, o2h, nullptr, nullptr, st))) return rc;
     k_metric_reduce<<<B, 256, sizeof(float) * 6 * T, st>>>(obj_pred, body_jtr, body, obj_gt, body_jtr_gt, body_gt, o2h, out, T, B, J, P, Db);
+    LAUNCH_CHECK(h);
+    return IDB_OK;
+}
+
+// ---- skeleton model metrics (eval_skeleton.py:46-68 calc_metric_single, train_diffusion_skeleton.py:65-87 calc_metric) -----
+namespace {
+// One block per sample b, read straight from the sample layout (B,1,C,T), C = 3 J + 3 P + 7 = [joints | keypoints | trans(3),
+// quat xyzw(4)]: per-frame terms by warps (lanes over joints / keypoints) for the future frames t >= past_len, then a sequential
+// mean over those frames.  out[k][b], k = mpjpe_h, mpjpe_o, translation_error, rotation_error (sign-min of the quaternion L1
+// distance, eval_skeleton.py:59-62), rotation_error_l2 (the same with the L2 norm, train_diffusion_skeleton.py:78-81).
+__global__ void __launch_bounds__(256)
+k_skeleton_metrics(const float* __restrict__ pred, const float* __restrict__ gt, float* __restrict__ out, int B, int T, int P0, int J, int Np) {
+    extern __shared__ float sm[];          // [5][nF] per-frame terms
+    const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int C = 3 * (J + Np) + 7, nF = T - P0;
+    const float* pp = pred + (size_t)b * C * T;
+    const float* gg = gt + (size_t)b * C * T;
+    auto dist3 = [&](int c0, int t) {
+        const float dx = pp[(size_t)c0 * T + t] - gg[(size_t)c0 * T + t], dy = pp[(size_t)(c0 + 1) * T + t] - gg[(size_t)(c0 + 1) * T + t],
+                    dz = pp[(size_t)(c0 + 2) * T + t] - gg[(size_t)(c0 + 2) * T + t];
+        return sqrtf(dx * dx + dy * dy + dz * dz);
+    };
+    for (int f = warp; f < nF; f += 8) {
+        const int t = P0 + f;
+        float sh = 0.f, so = 0.f;
+        for (int j = lane; j < J; j += 32) sh += dist3(3 * j, t);
+        for (int p = lane; p < Np; p += 32) so += dist3(3 * (J + p), t);
+        sh = warp_sum(sh); so = warp_sum(so);
+        if (lane == 0) {
+            const int c0 = 3 * (J + Np);
+            sm[0 * nF + f] = sh / (float)J;
+            sm[1 * nF + f] = so / (float)Np;
+            sm[2 * nF + f] = dist3(c0, t);
+            float e1 = 0.f, e2 = 0.f, s1 = 0.f, s2 = 0.f;
+            for (int k = 0; k < 4; k++) {
+                const float p = pp[(size_t)(c0 + 3 + k) * T + t], g = gg[(size_t)(c0 + 3 + k) * T + t];
+                const float dm = p - g, dp = p + g;
+                e1 += fabsf(dm); e2 += fabsf(dp); s1 += dm * dm; s2 += dp * dp;
+            }
+            sm[3 * nF + f] = fminf(e1, e2);
+            sm[4 * nF + f] = fminf(sqrtf(s1), sqrtf(s2));
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < 5) {
+        float s = 0.f;
+        for (int f = 0; f < nF; f++) s += sm[threadIdx.x * nF + f];
+        out[(size_t)threadIdx.x * B + b] = s / (float)nF;
+    }
+}
+}  // namespace
+
+extern "C" int idb_skeleton_metrics(idb_handle* h, int B, int T, int past_len, int n_joints, int n_points, const float* pred, const float* gt,
+                                    float* out, void* stream) {
+    IDB_ENTER(h);
+    if (!h || !pred || !gt || !out || B <= 0 || T <= 0 || n_joints <= 0 || n_points <= 0) return IDB_ERR_ARG;
+    if (past_len < 0 || past_len >= T) return idb_fail(h, IDB_ERR_ARG, "past_len must leave at least one future frame");
+    const int nF = T - past_len;
+    if (nF > 2048) return idb_fail(h, IDB_ERR_ARG, "at most 2048 future frames");
+    k_skeleton_metrics<<<B, 256, sizeof(float) * 5 * nF, (cudaStream_t)stream>>>(pred, gt, out, B, T, past_len, n_joints, n_points);
     LAUNCH_CHECK(h);
     return IDB_OK;
 }

@@ -293,6 +293,15 @@ class Engine:
         self._chk(self.lib.idb_encode_condition(self._h, B, Tp, self._ptr(past), self._ptr(pc), self._ptr(out), self._stream()))
         return out
 
+    def encode_condition_skeleton(self, past, zero_pose_obj):
+        """cond (Tp,B,256) of the skeleton model = conditioning encoder on the past frames (B,1,106,Tp) + the shape embedding
+        of zero_pose_obj (B,12,3) (reference skeleton MDM._get_embeddings); needs encoder.layers.* and shapeEmbedding.* loaded."""
+        past, zp = self._f32(past), self._f32(zero_pose_obj)
+        B, Tp = past.shape[0], past.shape[-1]
+        out = torch.empty(Tp, B, 256, device=self.device)
+        self._chk(self.lib.idb_encode_condition_skeleton(self._h, B, Tp, self._ptr(past), self._ptr(zp), self._ptr(out), self._stream()))
+        return out
+
     # ------------------------------------------------------------------ body model / geometry
     def load_body(self, smplh):
         f = lambda k: np.ascontiguousarray(np.asarray(smplh[k]), dtype=np.float32)
@@ -350,6 +359,20 @@ class Engine:
         self._chk(self.lib.idb_metrics(self._h, T, B, J, a[7].shape[1], a[2].shape[2], *[self._ptr(t) for t in a], self._ptr(out),
                                        self._stream()))
         return {k: out[i] for i, k in enumerate(self.METRIC_NAMES)}
+
+    SKELETON_METRIC_NAMES = ("mpjpe_h", "mpjpe_o", "translation_error", "rotation_error", "rotation_error_l2")
+
+    def skeleton_metrics(self, pred, gt, past_len, n_joints=21):
+        """The skeleton model's metrics (eval_skeleton.py:46-68; rotation_error_l2 = train_diffusion_skeleton.py:65-87) per sample
+        on the device: pred / gt (B,1,3 n_joints + 3 n_points + 7,T) -> dict of (B,) tensors, means over the frames t >= past_len."""
+        pred, gt = self._f32(pred), self._f32(gt)
+        B, _, Cn, T = pred.shape
+        if gt.shape != pred.shape or (Cn - 7 - 3 * n_joints) % 3 or Cn - 7 - 3 * n_joints <= 0:
+            raise EngineError("pred / gt must both be (B,1,3 n_joints + 3 n_points + 7,T)")
+        out = torch.empty(5, B, device=self.device)
+        self._chk(self.lib.idb_skeleton_metrics(self._h, B, T, int(past_len), int(n_joints), (Cn - 7 - 3 * n_joints) // 3, self._ptr(pred),
+                                                self._ptr(gt), self._ptr(out), self._stream()))
+        return {k: out[i] for i, k in enumerate(self.SKELETON_METRIC_NAMES)}
 
     def rollout_next_window(self, body, obj, jtr, T, past_len):
         """get_batch of eval_smpl_long.py:26-84 on the device: (gt (B,1,144,T), centroid (B,3)) of the next window from the

@@ -1,7 +1,10 @@
 """Host-side mirror of reference model/diffusion_skeleton.py (skeleton MDM :15-257; factory
 :259-299): 21 body joints + 12 object keypoints + 7-D object pose (106 channels).  The object
 keypoints of the prediction are re-derived from the predicted pose inside the library
-(calc_obj_pred :218-229)."""
+(calc_obj_pred :218-229).  _get_embeddings (:194-215) assembles `gt` on the host and runs the
+conditioning encoder (shape embedding, past-frame embeddings, positional encoding, 8 layers) in
+the library (`idb_encode_condition_skeleton`)."""
+import torch
 import torch.nn as nn
 
 from .diffusion_smpl import _EngineHost, _layer_stack, create_gaussian_diffusion  # noqa: F401
@@ -28,8 +31,19 @@ class MDM(_EngineHost, nn.Module):
         self.bodyFinalLinear = nn.Linear(D, args.smpl_dim)
         self.objFinalLinear = nn.Linear(D, 7)
 
+    def encode_condition(self, past, zero_pose_obj):
+        """cond (past_len,B,D) from the past frames (B,1,106,past_len) and the canonical object keypoints (B,12,3), on the
+        device (the part of `_get_embeddings` after the `gt` concatenation, reference :203-213)."""
+        return self.engine_for(past.device).encode_condition_skeleton(past, zero_pose_obj)
+
     def _get_embeddings(self, body_gt, obj_gt, pose_gt, zero_pose_obj):
-        raise NotImplementedError("the conditioning encoder is the next row of the hot-path table (SURVEY.md 8f)")
+        """Reference :194-215: body_gt (T,B,21,3) joints, obj_gt (T,B,12,3) keypoints, pose_gt (T,B,7), zero_pose_obj (B,12,3)
+        -> (embedding (past_len,B,D), gt (T,B,106)).  gt is the reference's concatenation; the encoder runs in the library."""
+        T, B, n_joints, _ = body_gt.shape
+        n_points = obj_gt.shape[2]
+        gt = torch.cat([body_gt.reshape(T, B, n_joints * 3), obj_gt.reshape(T, B, n_points * 3), pose_gt], dim=2)
+        past = gt[: self.args.past_len].permute(1, 2, 0).unsqueeze(1).contiguous()          # (B,1,106,past_len)
+        return self.encode_condition(past, zero_pose_obj), gt
 
     def forward(self, x, timesteps, zero_pose_obj, y=None):
         """x (B,1,106,T); zero_pose_obj (B,12,3) (reference :250-257)."""

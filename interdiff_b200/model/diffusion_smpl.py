@@ -29,8 +29,8 @@ class _EngineHost:
     rotary = "absolute"   # local-attention <= 1.5 rotary placement; 'bucketed' for >= 1.6 (SURVEY 8c)
 
     def _hot_state(self):
-        keep = ("decoder.", "encoder.", "pcEmbedding.", "bodyEmbedding.", "objEmbedding.", "bodyFinalLinear.", "objFinalLinear.",
-                "embedTimeStep.time_embed.", "PositionalEmbedding.pe")
+        keep = ("decoder.", "encoder.", "pcEmbedding.", "shapeEmbedding.", "bodyEmbedding.", "objEmbedding.", "bodyFinalLinear.",
+                "objFinalLinear.", "embedTimeStep.time_embed.", "PositionalEmbedding.pe")
         return {k: v for k, v in self.state_dict().items() if k.startswith(keep)}
 
     def _signature(self):

@@ -107,6 +107,29 @@ class FusedCorrection:
         return eng.correction_apply(x, y["inpainted_motion"], ti)
 
 
+class FusedSkeletonCorrection:
+    """The skeleton model's denoised_fn hook (eval_skeleton.py:80-111) as an object the diffusion recognises, the counterpart
+    of FusedCorrection: with it p_sample_loop keeps eval_skeleton's whole loop, including the correction steps, inside the
+    library.  Called directly (x, t, model_kwargs) it applies the same gate and runs the fused hook on x in place, so it also
+    works as a plain denoised_fn callback.
+
+    model_kwargs must carry what the reference's hook reads: y['inpainted_motion'] (B,1,106,T), y['obj_model'] (object with
+    .model = interdiff_b200 skeleton ObjProjector) and zero_pose_obj (B,12,3), which is bound together with the denoiser."""
+    is_fused_correction = True
+
+    def bind(self, eng, model_kwargs):
+        model_kwargs["y"]["obj_model"].model.load_into(eng)
+        return eng
+
+    def __call__(self, x, t, model_kwargs):
+        ti = int(t[0])
+        if ti > 500 or ti % 50 != 0:
+            return x
+        proj = model_kwargs["y"]["obj_model"].model
+        eng = proj.engine_for(x.device)
+        return eng.skeleton_correction_apply(x, model_kwargs["y"]["inpainted_motion"], model_kwargs["zero_pose_obj"], ti)
+
+
 def sample_postprocess(engine, sample, hand_pose, betas, past_len=10, future_len=None):
     """Tail of sample_once(_proj) (eval_smpl_short.py:154-173): 6D -> axis-angle and SMPL-H LBS of
     all T*B frames.  Returns body pose (T,B,159), object pose (T,B,6), verts (T,B,V,3), joints."""

@@ -68,6 +68,15 @@ def mdm_encoder_shapes(variant="smpl", D=256, F=None, n_layers=8, N=10):
     return s
 
 
+def mdm_skeleton_encoder_shapes(D=256, F=256, n_layers=8, N=10, n_points=12):
+    """Conditioning path of the skeleton model (model/diffusion_skeleton.py:194-215): the 8 encoder layers (d_ff 256) and
+    shapeEmbedding, the Linear on the flattened canonical object keypoints."""
+    s = mdm_encoder_shapes("skeleton", D=D, F=F, n_layers=n_layers, N=N)
+    s["shapeEmbedding.weight"] = (D, 3 * n_points)
+    s["shapeEmbedding.bias"] = (D,)
+    return s
+
+
 def pointnet_shapes(prefix="pcEmbedding."):
     """PointNet2Encoder(c_in=1, c_out=256, num_keypoints=1) (model/layers.py:111-141): two MSG set-abstraction
     modules (Conv2d 1x1 without bias + BatchNorm2d + ReLU, three times per scale) and the Linear head."""
@@ -154,7 +163,8 @@ def load_ref_weights(name, directory=None):
 def bench_weights(name, seed=233):
     """{state_dict name: torch tensor} for the benchmarks / probes / smoke run: the exported checkpoint tensors when
     weights_ref/<name>.npz exists, else seeded random init of the same shapes (the sinusoid tables are always rebuilt).
-    name: diffusion_smpl | diffusion_skeleton | correction_smpl | diffusion_smpl_encoder."""
+    name: diffusion_smpl | diffusion_skeleton | correction_smpl | correction_skeleton | diffusion_smpl_encoder |
+    diffusion_skeleton_encoder (the encoder names only; merge with diffusion_skeleton for a whole model)."""
     import torch
     sd = load_ref_weights(name)
     if sd is None:
@@ -164,12 +174,14 @@ def bench_weights(name, seed=233):
             shapes = projector_skeleton_shapes()
         elif name == "diffusion_smpl_encoder":
             shapes = {**mdm_encoder_shapes("smpl"), **pointnet_shapes()}
+        elif name == "diffusion_skeleton_encoder":
+            shapes = mdm_skeleton_encoder_shapes()
         else:
             variant = name[len("diffusion_"):]
             shapes = {k: v for k, v in mdm_hot_shapes(variant, F=1024 if variant == "smpl" else 256).items() if not k.endswith(".pe")}
         sd = random_state_dict(shapes, seed)
     sd = dict(sd)
-    if name.startswith("diffusion_") and name != "diffusion_smpl_encoder":
+    if name.startswith("diffusion_") and not name.endswith("_encoder"):
         pe = synthetic.sinusoid_table(5000, 256).reshape(5000, 1, 256)
         sd["PositionalEmbedding.pe"] = pe
         sd["embedTimeStep.sequence_pos_encoder.pe"] = pe
